@@ -550,6 +550,9 @@ def run_workload(args, name, wl, dev, rank, world, R, primary):
             off += g.numel()
         torch._foreach_copy_(grads, views)
 
+    dump = primary and args.dump_outputs is not None
+    last = {}
+
     def step(x, y):
         logits = model(x)
         loss = crit(logits, y)
@@ -564,6 +567,8 @@ def run_workload(args, name, wl, dev, rank, world, R, primary):
             o.step()
         if sharded:
             model.finish_step()
+        if dump:
+            last["logits"], last["loss"] = logits.detach(), loss.detach()
         return loss
 
     pool = make_batches(dims, b, args.pool, 2023 + rank, torch.int32, args.ids)
@@ -599,6 +604,7 @@ def run_workload(args, name, wl, dev, rank, world, R, primary):
     l0 = _lib.load().rsb_launch_count()
     ms_total = timed(lambda i: step(*dev_pool[i % len(dev_pool)]), steps)
     launches = _lib.load().rsb_launch_count() - l0
+    outputs = snapshot_outputs(model, last) if dump else None
     # per-kernel CUDA-event timing in a SEPARATE pass of the same steps (an event pair around every C call keeps
     # consecutive kernels from overlapping their launch latency, so it must not sit inside the `value` region)
     timer = RF.KernelTimer()
@@ -733,7 +739,41 @@ def run_workload(args, name, wl, dev, rank, world, R, primary):
     res["kernels"] = {k: {"calls_per_step": r["calls"] / ksteps, "ms_avg": round(r["ms_avg"], 4),
                           "share_of_step": round(r["ms_total"] / ms_kpass, 4)} for k, r in kern.items()}
     res["_objects"] = (model, opts, crit, cfg, dev_pool, pool)
+    res["_outputs"] = outputs
     return res
+
+
+DUMP_MAX_ELEMENTS = 1 << 20      # per array: at most 4 MB of float32
+
+
+def snapshot_outputs(model, last):
+    """What the last timed step handed back: its loss and logits, and the model's parameters and floating-point
+    buffers as the optimizer step left them.  An array of more than DUMP_MAX_ELEMENTS keeps a fixed, seeded
+    sample of its rows (sorted row ids, the same for every run of the same shape)."""
+    import torch
+
+    out = {"loss": last["loss"].float().reshape(1), "logits": last["logits"].float()}
+    tensors = list(model.named_parameters()) + [(n, b) for n, b in model.named_buffers() if b.is_floating_point()]
+    for name, t in tensors:
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            keep = max(1, DUMP_MAX_ELEMENTS // max(1, t[0].numel()))
+            g = torch.Generator().manual_seed(0)
+            rows = torch.randperm(t.shape[0], generator=g)[:keep].sort().values
+            t = t[rows.to(t.device)]
+        out[name] = t.float()
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(outputs, out_dir, max_bytes=64 << 20):
+    import numpy as np
+
+    total = sum(a.nbytes for a in outputs.values())
+    if total > max_bytes:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {max_bytes}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def sharded_parity_check(dims, dev, rank, world, R):
@@ -840,6 +880,9 @@ def main_ours(args, wl):
             parity = {"ok": False, "error": f"{type(exc).__name__}: {exc}"[:300]}
     res = run_workload(args, args.workload, wl, dev, rank, world, R, primary=True)
     model, opts, crit, cfg, dev_pool, pool = res.pop("_objects")
+    outputs = res.pop("_outputs")
+    if outputs is not None and rank == 0:
+        write_outputs(outputs, args.dump_outputs)
     dims, b = wl["dims"], args.batch
 
     # ---- reference-yaml batch (2048): launch-bound -> whole step captured in a CUDA graph -------------
@@ -868,6 +911,7 @@ def main_ours(args, wl):
             try:
                 r = run_workload(args, other, WORKLOADS[other], dev, rank, world, R, primary=False)
                 r.pop("_objects")
+                r.pop("_outputs")
                 r.pop("kernels", None)
                 if other == "deepfm_qr_criteo" and args.small_batch > 0:
                     try:
@@ -967,6 +1011,10 @@ def main():
     ap.add_argument("--no-torch-eager", action="store_true", help="skip the torch-eager-on-GPU comparison leg")
     ap.add_argument("--small-batch", type=int, default=2048,
                     help="also time this (reference yaml) batch eagerly and as one CUDA graph; 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, logits and model state after the last timed step as DIR/<name>.npy "
+                         "(float32; arrays over 2^20 elements as a seeded row sample), so that two builds can be "
+                         "compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = WORKLOADS[args.workload]
@@ -979,4 +1027,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the tree bench.py runs from may be read-only: no __pycache__ written into it
     main()

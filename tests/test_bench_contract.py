@@ -6,6 +6,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -51,6 +52,26 @@ def test_synthetic_id_generators():
     assert z[:, 2].unique().numel() < x[:, 2].unique().numel()          # far more duplicates than uniform ids
     again = bench.make_batches(dims, 8192, 1, 2023, torch.int64, "zipf")[0][0]
     assert torch.equal(z, again)                                        # seeded
+
+
+def test_dump_outputs_snapshot_is_seeded_float_and_bounded(tmp_path):
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Embedding(bench.DUMP_MAX_ELEMENTS // 4 + 3, 8), torch.nn.BatchNorm1d(8))
+    last = {"logits": torch.randn(64), "loss": torch.tensor(0.5)}
+    a = bench.snapshot_outputs(model, last)
+    b = bench.snapshot_outputs(model, last)
+    assert set(a) == {"loss", "logits", "0.weight", "1.weight", "1.bias", "1.running_mean", "1.running_var"}
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert a["loss"].shape == (1,) and a["logits"].shape == (64,)
+    table = model[0].weight.detach().numpy()
+    assert a["0.weight"].shape == (bench.DUMP_MAX_ELEMENTS // 8, 8)
+    assert np.array_equal(a["0.weight"], b["0.weight"])                   # the same rows every time
+    rows = [int(np.flatnonzero((table == r).all(1))[0]) for r in a["0.weight"][:5]]
+    assert rows == sorted(rows)
+    bench.write_outputs(a, str(tmp_path / "out"))
+    assert np.array_equal(np.load(tmp_path / "out" / "0.weight.npy"), a["0.weight"])
+    with pytest.raises(RuntimeError):
+        bench.write_outputs(a, str(tmp_path / "small"), max_bytes=1024)
 
 
 def test_workload_table_matches_the_survey_shapes():
