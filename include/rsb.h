@@ -497,7 +497,10 @@ RSB_API int rsb_lookup_fwd_sharded(const void* idx, int32_t idx_is_i32, const in
  *   aux_shards   [G]  the per-row aux array: PEP `s` for aux_mode FEATURE [N,1] / FEATURE_DIM [N,D] (fp32), the retrain
  *                     mask [N,D] (uint8) for MASK; NULL for every other kind / mode.
  * Replicated on every rank, passed as for rsb_lookup_fwd: table1 (QR emb1), aux for PEP GLOBAL / DIMENSION and the
- * OPTEMBED thresholds, fc_replicated [n_global], bias.  Arguments not listed here are those of rsb_lookup_fwd. */
+ * OPTEMBED per-field thresholds t [F] (NULL = mask-E off), fc_replicated [n_global], bias.  OPTEMBED's mask_d_idx is
+ * this rank's own [B, F] draw, one index per lookup, as for rsb_lookup_fwd.  Arguments not listed here are those of
+ * rsb_lookup_fwd.  The OptEmbed eval cache (rsb_optembed_eval_weight run on each rank's weight shard) is gathered with
+ * kind = VANILLA over the eval shards. */
 RSB_API int rsb_lookup_fwd_sharded_kind(int32_t kind, const void* idx, int32_t idx_is_i32, const int64_t* offsets, int64_t B,
                                         int32_t F, int32_t D, const float* const* table_shards, int32_t G, int64_t n_rows,
                                         int64_t n_global, const float* table1, int64_t divider, const void* aux,
@@ -507,7 +510,8 @@ RSB_API int rsb_lookup_fwd_sharded_kind(int32_t kind, const void* idx, int32_t i
 /* rsb_lookup_bwd_rows over the same shards (the variants' chain rules re-read the table / threshold / mask rows from
  * their owners); the per-lookup gradients rg_main / rg_aux stay local and are then pushed to the owners with
  * rsb_segment_scatter_shards (main table; PEP `s` with its own gradient shards), the replicated parameters' gradients
- * are reduced locally (rsb_small_table_grad for emb1) and averaged by the caller's allreduce. */
+ * are reduced locally (rsb_small_table_grad for emb1; OPTEMBED: g_t[f] = -sum_b rg_aux[b, f] over the [B, F]
+ * per-lookup scalars, with t replicated and the forward's mask_d_idx) and averaged by the caller's allreduce. */
 RSB_API int rsb_lookup_bwd_rows_sharded(int32_t kind, const int64_t* rows, int64_t B, int32_t F, int32_t D,
                                         const float* const* table_shards, int32_t G, int64_t n_rows, const float* table1,
                                         int64_t divider, const void* aux, const void* const* aux_shards, int32_t aux_mode,

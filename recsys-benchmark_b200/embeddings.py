@@ -420,6 +420,16 @@ class OptEmbed(IOptEmbed):
     def get_weight(self, mask_d: Optional[torch.Tensor] = None):
         """Masked full table (deepfm_opt_embed.py:148-202).  mask_d: int indices per field /
         per feature (dims 0..k kept) or a [N,D] bool mask."""
+        rows_idx, bool_mask = self._mask_d_rows(mask_d)
+        out, _ = self._masked_table(rows_idx)
+        if bool_mask is not None:
+            out = out * bool_mask.to(out.dtype)
+        self._cur_weight = out
+        return self._cur_weight
+
+    def _mask_d_rows(self, mask_d: Optional[torch.Tensor]):
+        """get_weight's mask-D as (per-row int64 [N] indices or None, [N, D] bool mask or None); in training without
+        a mask_d, the reference's random draw."""
         device = self._weight.device
         rows_idx = None
         bool_mask = None
@@ -437,11 +447,7 @@ class OptEmbed(IOptEmbed):
                                                        output_size=self._num_item)
             else:
                 bool_mask = mask_d.to(device)
-        out, _ = self._masked_table(rows_idx.contiguous() if rows_idx is not None else None)
-        if bool_mask is not None:
-            out = out * bool_mask.to(out.dtype)
-        self._cur_weight = out
-        return self._cur_weight
+        return (rows_idx.contiguous() if rows_idx is not None else None), bool_mask
 
     def _spec(self):
         return RF.LookupSpec(L.KIND_OPTEMBED, self._num_item, self._hidden_size, aux_mode=self._norm, module=self)
@@ -507,20 +513,20 @@ class OptEmbed(IOptEmbed):
         return (emb.abs().sum(1) > 0).to(torch.int64).cpu()
 
     def get_submask(self) -> torch.Tensor:
-        if self._submask_cache is not None:
-            return self._submask_cache
+        if self._submask_cache is None:
+            self._submask_cache = self._submask(self.get_mask_e)
+        return self._submask_cache
+
+    def _submask(self, get_mask_e) -> torch.Tensor:
+        """get_submask without the cache, from the mask-E that `get_mask_e()` returns."""
         if isinstance(self._mask_e_module, nn.Identity):
-            res = self._field_dims if self._mode_d == "field" else torch.ones(self._num_item, dtype=torch.int64)
-        else:
-            mask_e = self.get_mask_e()
-            if self._mode_d == "feature":
-                res = mask_e
-            else:
-                num_e = torch.cat([torch.zeros(1, dtype=torch.int64), mask_e.cumsum(0)])
-                offsets = torch.cat([torch.zeros(1, dtype=torch.int64), self._field_dims]).cumsum(0)
-                res = num_e[offsets[1:]] - num_e[offsets[:-1]]
-        self._submask_cache = res
-        return res
+            return self._field_dims if self._mode_d == "field" else torch.ones(self._num_item, dtype=torch.int64)
+        mask_e = get_mask_e()
+        if self._mode_d == "feature":
+            return mask_e
+        num_e = torch.cat([torch.zeros(1, dtype=torch.int64), mask_e.cumsum(0)])
+        offsets = torch.cat([torch.zeros(1, dtype=torch.int64), self._field_dims]).cumsum(0)
+        return num_e[offsets[1:]] - num_e[offsets[:-1]]
 
 
 class RetrainOptEmbed(IOptEmbed):

@@ -30,7 +30,7 @@ from . import _lib as L
 from . import functional as RF
 from .dcn import DCN_Mix
 from .deepfm import DeepFM
-from .embeddings import IEmbedding
+from .embeddings import IEmbedding, OptEmbed, RetrainOptEmbed
 from .linalg import run_sequential
 
 
@@ -151,10 +151,11 @@ def _open(handle: bytes, device) -> int:
 
 class ShardGroup:
     """The per-rank buffers (table shard and its gradient accumulator; optionally a per-row aux array - PEP thresholds
-    or a retrain mask - and its gradient accumulator) and the device-resident pointer tables to every rank's copy."""
+    or a retrain mask - and its gradient accumulator; optionally an `eval` shard [n_local, dim] - OptEmbed's cached
+    masked table) and the device-resident pointer tables to every rank's copy."""
 
     def __init__(self, num_rows: int, dim: int, device: torch.device, group=None, aux_cols: int = 0,
-                 aux_is_mask: bool = False, aux_grad: bool = False):
+                 aux_is_mask: bool = False, aux_grad: bool = False, eval_table: bool = False):
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -170,6 +171,8 @@ class ShardGroup:
             self.buf["aux"] = SharedBuffer(shape, device)
             if aux_grad:
                 self.buf["aux_grad"] = SharedBuffer((self.n_local, aux_cols), device)
+        if eval_table:
+            self.buf["eval"] = SharedBuffer((self.n_local, dim), device)
         names = tuple(self.buf)
         handles = {k: self.buf[k].handle() for k in names}
         if self.world > 1:
@@ -420,14 +423,16 @@ class _ShardedKindLookup(torch.autograd.Function):
     """_ShardedLookup for the lightweight variants (SURVEY 8e): the MAIN table (PEP / masked weight, QR emb2) and the
     per-row aux array (PEP `s` of the feature / feature_dim kinds, retrain masks) are read from the owners' shards inside
     the gather and inside the backward's chain-rule kernel; their gradients are pre-reduced per unique row and pushed
-    into the owners' accumulators.  Small parameters (QR emb1, PEP global / dimension thresholds, fc, bias) are
-    replicated: their gradients go back to autograd and are averaged with the other replicated gradients.
+    into the owners' accumulators.  Small parameters (QR emb1, PEP global / dimension thresholds, OptEmbed's per-field
+    thresholds `t`, fc, bias) are replicated: their gradients go back to autograd and are averaged with the other
+    replicated gradients.  `mask_d` (OptEmbed) is the [B, F] int64 mask-D draw of this rank's lookups.
     `table` (this rank's shard) is an input only so that autograd runs the backward; its gradient is never returned."""
 
     @staticmethod
-    def forward(ctx, sg: ShardGroup, spec, x, offsets, table, table1, aux_rep, fc, bias, presort, amax_slots):
+    def forward(ctx, sg: ShardGroup, spec, x, offsets, table, table1, aux_rep, fc, bias, presort, amax_slots,
+                mask_d=None):
         lib = L.load()
-        dev = L.require_cuda(x, offsets, table, table1, aux_rep, fc, bias)
+        dev = L.require_cuda(x, offsets, table, table1, aux_rep, fc, bias, mask_d)
         x = x.contiguous()
         b, f = x.shape
         e = spec.row_width
@@ -437,16 +442,17 @@ class _ShardedKindLookup(torch.autograd.Function):
         s = torch.empty(b, e, dtype=torch.float32, device=dev) if use_fm else None
         rows = torch.empty(b, f, dtype=torch.int64, device=dev)
         aux_sh = sg.ptrs.get("aux")
-        nbytes = b * (f * x.element_size() + 2 * f * e * 4 + f * 8 + (f * 4 + 4 + e * 4 if use_fm else 0))
+        md_bytes = RF._aux_row_bytes(spec, f, mask_d) if mask_d is not None else 0
+        nbytes = b * (f * x.element_size() + 2 * f * e * 4 + f * 8 + md_bytes + (f * 4 + 4 + e * 4 if use_fm else 0))
         RF._call("lookup_fwd_sharded", lib.rsb_lookup_fwd_sharded_kind, spec.kind, L.ptr(x), int(x.dtype == torch.int32),
                  L.ptr(offsets), b, f, spec.dim, L.ptr(sg.ptrs["table"]), sg.world, sg.num_rows, spec.num_global,
-                 L.ptr(table1), spec.divider, L.ptr(aux_rep), L.ptr(aux_sh), spec.aux_mode, None,
+                 L.ptr(table1), spec.divider, L.ptr(aux_rep), L.ptr(aux_sh), spec.aux_mode, L.ptr(mask_d),
                  L.ptr(fc) if use_fm else None, L.ptr(bias) if use_fm else None, L.ptr(emb), L.ptr(y), L.ptr(s),
                  L.ptr(rows), L.ptr(sg.err_flag), L.ptr(amax_slots), L.stream_ptr(dev), nbytes=nbytes)
         ctx.sg, ctx.spec, ctx.use_fm, ctx.shape = sg, spec, use_fm, (b, f)
         ctx.fc_shape = tuple(fc.shape) if fc is not None else None
         ctx.presorted = RF.early_sort(rows, sg.num_rows, key_div=spec.divider if spec.is_qr else 0) if presort else None
-        ctx.save_for_backward(rows, emb, s, table1, aux_rep)
+        ctx.save_for_backward(rows, emb, s, table1, aux_rep, mask_d)
         ctx.mark_non_differentiable(rows)
         return emb, (y if use_fm else emb.new_empty(0)), rows
 
@@ -455,13 +461,14 @@ class _ShardedKindLookup(torch.autograd.Function):
         lib = L.load()
         sg: ShardGroup = ctx.sg
         spec = ctx.spec
-        rows, emb, s, table1, aux_rep = ctx.saved_tensors
+        rows, emb, s, table1, aux_rep, mask_d = ctx.saved_tensors
         b, f = ctx.shape
         e = spec.row_width
         n = b * f
         dev = rows.device
         kind = spec.kind
-        need = ctx.needs_input_grad   # (sg, spec, x, offsets, table, table1, aux_rep, fc, bias, presort, amax_slots)
+        # (sg, spec, x, offsets, table, table1, aux_rep, fc, bias, presort, amax_slots, mask_d)
+        need = ctx.needs_input_grad
         use_gy = ctx.use_fm and g_y is not None and g_y.numel() == b
         g_emb = g_emb.contiguous() if g_emb is not None else None
         g_y = g_y.contiguous() if use_gy else None
@@ -475,12 +482,16 @@ class _ShardedKindLookup(torch.autograd.Function):
             rg_main = torch.empty(n, e, dtype=torch.float32, device=dev)
             if kind == L.KIND_QR_MULT or (kind == L.KIND_PEP and (per_row_s or need[6])):
                 rg_aux = torch.empty(n, e, dtype=torch.float32, device=dev)
-            n_out = 2 if rg_aux is not None else 1
-            nbytes = b * (f * 8 + f * e * 4 * (1 + int(use_gy)) + n_out * f * e * 4 + (e * 4 + 4 if use_gy else 0))
+            elif kind == L.KIND_OPTEMBED and aux_rep is not None and need[6]:
+                rg_aux = torch.empty(b, f, dtype=torch.float32, device=dev)     # one g_z per lookup
+            n_out = 2 if (rg_aux is not None and kind != L.KIND_OPTEMBED) else 1
+            md_bytes = RF._aux_row_bytes(spec, f, mask_d) if mask_d is not None else 0
+            nbytes = b * (f * 8 + f * e * 4 * (1 + int(use_gy)) + n_out * f * e * 4 + md_bytes
+                          + (e * 4 + 4 if use_gy else 0))
             RF._call("lookup_bwd_rows", lib.rsb_lookup_bwd_rows_sharded, kind, L.ptr(rows), b, f, spec.dim,
                      L.ptr(sg.ptrs["table"]), sg.world, sg.num_rows, L.ptr(table1), spec.divider, L.ptr(aux_rep),
-                     L.ptr(aux_sh), spec.aux_mode, None, L.ptr(emb), L.ptr(s), L.ptr(g_y), L.ptr(g_emb), L.ptr(rg_main),
-                     L.ptr(rg_aux), L.stream_ptr(dev), nbytes=nbytes)
+                     L.ptr(aux_sh), spec.aux_mode, L.ptr(mask_d), L.ptr(emb), L.ptr(s), L.ptr(g_y), L.ptr(g_emb),
+                     L.ptr(rg_main), L.ptr(rg_aux), L.stream_ptr(dev), nbytes=nbytes)
             if kind == L.KIND_QR_ADD:
                 rg_aux = rg_main
         # ---- stage 2: sorted, pre-reduced per unique row, pushed to the owner ----
@@ -504,6 +515,8 @@ class _ShardedKindLookup(torch.autograd.Function):
                 push(rg_aux.sum(dim=1, keepdim=True).contiguous(), 1, "aux_grad")
         elif kind == L.KIND_PEP and need[6]:
             g_aux = rg_aux.sum(dim=0) if spec.aux_mode == L.PEP_DIMENSION else rg_aux.sum().reshape(1)
+        elif kind == L.KIND_OPTEMBED and rg_aux is not None:
+            g_aux = -rg_aux.sum(dim=0)               # as the single-device backward: g_t[f] = -sum_b g_z[b, f]
         if spec.is_qr and need[5]:
             g_table1 = (RF.small_table_grad(rows, rg_aux, table1.shape[0], key_mod=spec.divider)
                         if (not RF.DETERMINISTIC or table1.shape[0] <= 32) else None)
@@ -513,38 +526,58 @@ class _ShardedKindLookup(torch.autograd.Function):
             if need[7]:
                 g_fc = RF.fc_grad(rows, g_y, b, f, ctx.fc_shape, spec.num_global, None if spec.is_qr else (skeys, perm))
             g_bias = g_y.sum().reshape(1)
-        return None, None, None, None, None, g_table1, g_aux, g_fc, g_bias, None, None
+        return None, None, None, None, None, g_table1, g_aux, g_fc, g_bias, None, None, None
+
+
+def _kernel_tensors(inner: IEmbedding):
+    """(main table, QR emb1, aux) as the module holds them.  The OptEmbed kinds' own _tensors() returns other things:
+    the supernet its eval cache outside training, the retrain module a uint8 copy of its mask (or an AssertionError
+    before init_mask); here they are the weight and `t` Parameters, resp. the weight and the `_mask` Parameter (None
+    before init_mask)."""
+    if isinstance(inner, OptEmbed):
+        return inner._weight, None, inner._t_param()
+    if isinstance(inner, RetrainOptEmbed):
+        return inner._weight, None, inner._mask
+    return inner._tensors()
 
 
 class ShardedEmbedding(IEmbedding):
     """Any of the per-row variants with its big arrays row-sharded over the process group (SURVEY 8e):
     QRHashingEmbedding mult / add (emb2 sharded, the <= divider-row emb1 replicated), PepEmbeeding (emb.weight sharded;
-    `s` sharded for the feature / feature_dim threshold types, replicated for global / dimension), RetrainPepEmbedding
+    `s` sharded for the feature / feature_dim threshold types, replicated for global / dimension), the OptEmbed
+    supernet (`_weight` sharded, the per-field thresholds `t` replicated, mask-D drawn per lookup), RetrainPepEmbedding
     and RetrainOptEmbed (weight and bool mask sharded).
 
     Built FROM the single-device module (`inner`, constructed the usual way - same seed on every rank - so its
     initialisation, kwargs and methods are the reference's): its big tensors are copied into this rank's IPC shard
     buffers and the module's own Parameters are re-pointed at them, so parameter names stay the reference's while
     their leading dimension becomes ceil(rows / G).  `load_full_state_dict` / `full_state_dict` convert from / to the
-    reference's single-device state dict."""
+    reference's single-device state dict.
 
-    KINDS = (L.KIND_QR_MULT, L.KIND_QR_ADD, L.KIND_PEP, L.KIND_MASK)
+    OptEmbed in eval mode gathers, like the reference, from a cached masked table: here one `eval` shard per rank,
+    rebuilt by every rank at the same point (a collective, between two barriers: nobody overwrites its shard while a
+    peer still reads it, and nobody gathers before every shard is rebuilt).  A training forward invalidates it."""
+
+    KINDS = (L.KIND_QR_MULT, L.KIND_QR_ADD, L.KIND_PEP, L.KIND_MASK, L.KIND_OPTEMBED)
 
     def __init__(self, inner: IEmbedding, group=None, device=None):
         super().__init__()
         spec = inner._spec()
         if spec.kind not in self.KINDS:
-            raise NotImplementedError("row sharding covers vanilla (ShardedVanillaEmbedding), QR mult / add, PEP and "
-                                      "masked-retrain tables")
+            raise NotImplementedError("row sharding covers vanilla (ShardedVanillaEmbedding), QR mult / add, PEP, "
+                                      "OptEmbed and masked-retrain tables")
         if inner._mode is not None or spec.sparse_grad or spec.modulus:
             raise NotImplementedError("sharded tables serve the dense-gradient [B,F,D] lookup only")
+        if isinstance(inner, OptEmbed) and inner._t_param() is not None and inner._mask_e_module.mode_threshold_e != "field":
+            raise NotImplementedError("sharded OptEmbed takes its mask-E thresholds per field (mode_threshold_e='field')")
         device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         inner = inner.to(device)
-        table, _table1, aux = inner._tensors()
+        table, _table1, aux = _kernel_tensors(inner)
         per_row = spec.kind == L.KIND_MASK or (spec.kind == L.KIND_PEP and spec.aux_mode in _PER_ROW_PEP)
-        self.shards = ShardGroup(table.shape[0], table.shape[1], device, group,
-                                 aux_cols=int(aux.shape[1]) if per_row else 0, aux_is_mask=spec.kind == L.KIND_MASK,
-                                 aux_grad=per_row and spec.kind == L.KIND_PEP)
+        aux_cols = (int(table.shape[1]) if spec.kind == L.KIND_MASK else int(aux.shape[1])) if per_row else 0
+        self.shards = ShardGroup(table.shape[0], table.shape[1], device, group, aux_cols=aux_cols,
+                                 aux_is_mask=spec.kind == L.KIND_MASK, aux_grad=per_row and spec.kind == L.KIND_PEP,
+                                 eval_table=spec.kind == L.KIND_OPTEMBED)
         self._per_row_aux = per_row
         self._full_rows = int(table.shape[0])
         self.inner = inner
@@ -552,73 +585,199 @@ class ShardedEmbedding(IEmbedding):
         with torch.no_grad():
             sg.buf["table"].tensor.copy_(shard_of_full(table.detach(), sg.rank, sg.world))
             table.data = sg.buf["table"].tensor
-            if per_row:
+            if isinstance(inner, RetrainOptEmbed):
+                if aux is not None:
+                    self._install_mask(aux.detach())
+            elif per_row:
                 sg.aux_tensor().copy_(shard_of_full(aux.detach(), sg.rank, sg.world))
                 aux.data = sg.aux_tensor()
         if hasattr(inner, "_nnz") and torch.is_tensor(inner._nnz):
             inner._nnz = inner._nnz.to(device)
+        if isinstance(inner, OptEmbed):
+            # the reference's eval cache: "fresh" (an empty table: eval() before any training or get_weight raises,
+            # as F.embedding does), "stale" (rebuilt on the next eval lookup) or "ready"
+            cur = inner._cur_weight
+            self._eval_state = "fresh" if cur is not None and cur.numel() == 0 else "stale"
+            inner._cur_weight = None if self._eval_state == "stale" else cur
 
     # -- what the step protocol of the sharded models needs -------------------------------
     def shard_params(self) -> List[torch.nn.Parameter]:
-        table, _t1, aux = self.inner._tensors()
+        table, _t1, aux = _kernel_tensors(self.inner)
         out = [table]
-        if self._per_row_aux and aux.requires_grad:
+        if self._per_row_aux and aux is not None and aux.requires_grad:
             out.append(aux)
         return out
 
     def expose_shard_grads(self, on: bool):
-        table, _t1, aux = self.inner._tensors()
+        table, _t1, aux = _kernel_tensors(self.inner)
         table.grad = self.shards.buf["table_grad"].tensor if on else None
         if "aux_grad" in self.shards.buf:
             aux.grad = self.shards.buf["aux_grad"].tensor if on else None
 
     # -- conversion from / to the reference's single-device tensors --------------------------
     def _names(self):
-        table, _t1, aux = self.inner._tensors()
-        big = {id(table): True}
-        if self._per_row_aux:
-            big[id(aux)] = True
-        return {n: id(p) in big for n, p in list(self.inner.named_parameters()) + list(self.inner.named_buffers())}
+        """{state-dict key: sharded?} over the module's persistent state (the reference's keys; OptEmbed's
+        non-persistent `_cur_weight` is not part of it)."""
+        table, _t1, aux = _kernel_tensors(self.inner)
+        big = {id(table)}
+        if self._per_row_aux and aux is not None:
+            big.add(id(aux))
+        return {n: id(t) in big for n, t in self.inner.state_dict(keep_vars=True).items()}
+
+    def _gather_full(self, local: torch.Tensor, num_rows: int) -> torch.Tensor:
+        """The full array of which every rank holds `local` (its rows, padded): an all-gather at world > 1."""
+        sg = self.shards
+        as_bytes = local.dtype == torch.bool
+        local = (local.view(torch.uint8) if as_bytes else local).contiguous()
+        if sg.world == 1:
+            parts = [local]
+        else:
+            parts = [torch.empty_like(local) for _ in range(sg.world)]
+            dist.all_gather(parts, local, group=sg.group)
+        full = full_from_shards(parts, num_rows)
+        return full.view(torch.bool) if as_bytes else full
+
+    def _all_sum(self, count: torch.Tensor) -> int:
+        """A device int64 count summed over the ranks."""
+        sg = self.shards
+        if sg.world > 1:
+            dist.all_reduce(count, group=sg.group)
+        return int(count.item())
+
+    @torch.no_grad()
+    def _install_mask(self, full: torch.Tensor):
+        """Keep this rank's rows of a full [N, D] retrain mask (any dtype, non-zero = kept) in the aux shard and point
+        the module's `_mask` at that shard; no full copy stays alive.  full_state_dict gives the mask back in `full`'s
+        dtype (RetrainOptEmbed.init_mask makes an int64 mask)."""
+        sg, inner = self.shards, self.inner
+        self._mask_dtype = full.dtype
+        m = sg.aux_tensor()
+        mine = full.to(sg.device)[sg.rank::sg.world]
+        m[: mine.shape[0]].copy_(mine != 0)
+        m[mine.shape[0]:] = False
+        inner._mask = nn.Parameter(m, requires_grad=False)
+        inner._cur_weight = None
+
+    def init_mask(self, mask_e: torch.Tensor, mask_d: torch.Tensor):
+        """RetrainOptEmbed.init_mask (deepfm_opt_embed.py:660-672) over the shards: the module builds the reference
+        mask, this rank keeps its rows.  Returns this rank's shard of the mask ([ceil(N / G), D] bool)."""
+        inner = self.inner
+        if not isinstance(inner, RetrainOptEmbed):
+            raise AttributeError(f"'{type(inner).__name__}' has no init_mask")
+        full = inner.init_mask(mask_e, mask_d)
+        self._install_mask(full.detach())
+        del full
+        return inner._mask
 
     @torch.no_grad()
     def load_full_state_dict(self, state: Dict[str, torch.Tensor]):
-        sg = self.shards
-        mine = dict(list(self.inner.named_parameters()) + list(self.inner.named_buffers()))
+        sg, inner = self.shards, self.inner
+        if isinstance(inner, RetrainOptEmbed) and inner._mask is None and "_mask" in state:
+            self._install_mask(state["_mask"])
+        mine = dict(list(inner.named_parameters()) + list(inner.named_buffers()))
         for name, sharded in self._names().items():
             src = state[name].to(sg.device)
             mine[name].copy_(shard_of_full(src, sg.rank, sg.world) if sharded else src)
+        if isinstance(inner, OptEmbed) and self._eval_state == "ready":
+            self._eval_state = "stale"
 
     @torch.no_grad()
     def full_state_dict(self) -> Dict[str, torch.Tensor]:
-        sg = self.shards
+        inner = self.inner
         out = {}
-        mine = dict(list(self.inner.named_parameters()) + list(self.inner.named_buffers()))
+        mine = dict(list(inner.named_parameters()) + list(inner.named_buffers()))
         for name, sharded in self._names().items():
             t = mine[name].detach()
             if not sharded:
                 out[name] = t.clone()
-                continue
-            as_bytes = t.dtype == torch.bool
-            local = (t.view(torch.uint8) if as_bytes else t).contiguous()
-            if sg.world == 1:
-                parts = [local]
             else:
-                parts = [torch.empty_like(local) for _ in range(sg.world)]
-                dist.all_gather(parts, local, group=sg.group)
-            full = full_from_shards(parts, self._full_rows)
-            out[name] = full.view(torch.bool) if as_bytes else full
+                full = self._gather_full(t, self._full_rows)
+                out[name] = full.to(self._mask_dtype) if isinstance(inner, RetrainOptEmbed) and name == "_mask" else full
         return out
 
+    # -- OptEmbed: the eval cache over the shards ----------------------------------------------
+    def _shard_rows(self, full_rows: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+        """This rank's rows of a global per-row array (zero padding: a zero weight row yields a zero masked row)."""
+        if full_rows is None:
+            return None
+        return shard_of_full(full_rows.to(self.shards.device), self.shards.rank, self.shards.world).contiguous()
+
     @torch.no_grad()
-    def get_weight(self):
+    def _rebuild_eval(self, mask_d: Optional[torch.Tensor]):
+        """OptEmbed.get_weight(mask_d) into this rank's `eval` shard: every row through rsb_optembed_eval_weight, the
+        kernel of the single-device cache, with the global per-row `t` and mask-D arrays sliced to this rank's rows.
+        Collective: all ranks rebuild at the same point (as validate_epoch does)."""
+        inner, sg = self.inner, self.shards
+        rows_idx, bool_mask = inner._mask_d_rows(mask_d)
+        t_sh = self._shard_rows(inner._t_rows())
+        md_sh = self._shard_rows(rows_idx)
+        out = sg.buf["eval"].tensor
+        dev = sg.device
+        sg.barrier()        # no peer still gathers from the shard about to be overwritten
+        RF._call("optembed_eval_weight", L.load().rsb_optembed_eval_weight, L.ptr(inner._weight), L.ptr(t_sh),
+                 L.ptr(md_sh), inner._norm, sg.n_local, sg.dim, L.ptr(out), None, L.stream_ptr(dev))
+        if bool_mask is not None:
+            out.mul_(self._shard_rows(bool_mask).to(out.dtype))
+        sg.barrier()        # every shard rebuilt before any peer gathers from it
+        self._eval_state = "ready"
+
+    def _eval_lookup(self, x, offsets, fc, bias, mask_d):
+        """OptEmbed.lookup outside training: the plain gather over the `eval` shards (rebuilt first when stale or when a
+        mask_d is given).  Not differentiable: the reference evaluates under no_grad."""
+        if self._eval_state != "ready" or mask_d is not None:
+            if self._eval_state == "fresh" and mask_d is None:
+                # reference behaviour on a fresh module in eval(): F.embedding on an empty weight
+                raise RuntimeError("'weight' must be 2-D")
+            self._rebuild_eval(mask_d)
+        sg = self.shards
+        lib = L.load()
+        dev = L.require_cuda(x, offsets, fc, bias)
+        if x.dtype not in (torch.int32, torch.int64):
+            raise RuntimeError(f"rsb: ids must be int32 or int64, got {x.dtype}")
+        x = x.contiguous()
+        b, f = x.shape
+        d = sg.dim
+        use_fm = fc is not None
+        emb = torch.empty(b, f, d, dtype=torch.float32, device=dev)
+        y = torch.empty(b, dtype=torch.float32, device=dev) if use_fm else None
+        s = torch.empty(b, d, dtype=torch.float32, device=dev) if use_fm else None
+        rows = torch.empty(b, f, dtype=torch.int64, device=dev)
+        slots = RF.amax_slots_for(dev)
+        nbytes = b * (f * x.element_size() + 2 * f * d * 4 + f * 8 + (f * 4 + 4 + d * 4 if use_fm else 0))
+        RF._call("lookup_fwd_sharded", lib.rsb_lookup_fwd_sharded_kind, L.KIND_VANILLA, L.ptr(x),
+                 int(x.dtype == torch.int32), L.ptr(offsets), b, f, d, L.ptr(sg.ptrs["eval"]), sg.world, sg.num_rows,
+                 sg.num_rows, None, 0, None, None, 0, None, L.ptr(fc) if use_fm else None,
+                 L.ptr(bias) if use_fm else None, L.ptr(emb), L.ptr(y), L.ptr(s), L.ptr(rows), L.ptr(sg.err_flag),
+                 L.ptr(slots), L.stream_ptr(dev), nbytes=nbytes)
+        if slots is not None:
+            emb._rsb_amax_slots = slots
+        return emb, y
+
+    @torch.no_grad()
+    def get_weight(self, mask_d: Optional[torch.Tensor] = None):
         """The effective [N, D] table the reference's get_weight returns (QR: emb1 (x) emb2, PEP: soft-thresholded,
-        retrain: weight * mask) = the lookup of every id; peer rows are read in place, no collective."""
+        retrain: weight * mask) = the lookup of every id; peer rows are read in place, no collective.  OptEmbed: the
+        masked table for `mask_d` (deepfm_opt_embed.py:148-202), rebuilt into the eval shards (which it leaves as the
+        eval cache, like the reference) and all-gathered - a collective.  The other kinds ignore mask_d, as
+        RetrainOptEmbed does."""
+        if isinstance(self.inner, OptEmbed):
+            self._rebuild_eval(mask_d)
+            return self._gather_full(self.shards.buf["eval"].tensor, self._full_rows)
         ids = torch.arange(self.inner._num_item, device=self.shards.device)
         return self(ids)
 
-    # -- the plugin's bookkeeping methods, global over the shards (the scripts call them: train_deepfm_pep.py:63,71) ------
+    def forward(self, x, mask_d=None):
+        """IEmbedding.forward; OptEmbed outside training rebuilds its eval cache with `mask_d` first (a collective), as
+        OptEmbed.forward does."""
+        if isinstance(self.inner, OptEmbed) and not self.training and mask_d is not None:
+            self._rebuild_eval(mask_d)
+        return self._plugin_forward(x)
+
+    # -- the plugin's bookkeeping methods, global over the shards (the scripts call them: train_deepfm_pep.py:63,71,
+    #    train_deepfm_optembed.py, SURVEY 8b) ------
     def __getattr__(self, name):
-        """Attributes of the wrapped module (`sparsity`, `checkpoint_weight_dir`, `threshold_type`, ...) read through."""
+        """Attributes of the wrapped module (`sparsity`, `checkpoint_weight_dir`, `threshold_type`, `get_l_s`, ...)
+        read through."""
         try:
             return super().__getattr__(name)
         except AttributeError:
@@ -626,6 +785,14 @@ class ShardedEmbedding(IEmbedding):
             if inner is None or name == "inner":
                 raise
             return getattr(inner, name)
+
+    def _optembed_count(self) -> int:
+        """Surviving weights of the mask-E-only table (OptEmbed.get_sparsity): the eval kernel's count on every shard,
+        all-reduced (padding rows are zero and count nothing)."""
+        inner = self.inner
+        _, cnt = RF.optembed_eval_weight(inner._weight.detach(), self._shard_rows(inner._t_rows()), None, inner._norm,
+                                         want_out=False, want_count=True)
+        return self._all_sum(cnt)
 
     def get_num_params(self) -> int:
         inner, sg = self.inner, self.shards
@@ -637,6 +804,12 @@ class ShardedEmbedding(IEmbedding):
                 dist.all_reduce(t, group=sg.group)
                 n = int(t.item())
             return n
+        if kind == L.KIND_OPTEMBED:
+            if self._eval_state == "ready" and not self.training:
+                return self._all_sum(torch.count_nonzero(sg.buf["eval"].tensor).reshape(1))
+            return self._optembed_count()
+        if isinstance(inner, RetrainOptEmbed):
+            return self._all_sum(torch.count_nonzero(inner._mask).reshape(1))
         if kind == L.KIND_MASK:
             return inner.get_num_params()                # counted on the full mask when the module was built
         sharded = self._names()
@@ -647,11 +820,33 @@ class ShardedEmbedding(IEmbedding):
 
     def get_sparsity(self, get_n_params=False):
         inner = self.inner
-        if inner._spec().kind != L.KIND_PEP:
-            return inner.get_sparsity(get_n_params)
-        total = self._full_rows * inner._hidden_size
-        n = self.get_num_params()
-        return ((1 - n / total), n) if get_n_params else 1 - n / total
+        kind = inner._spec().kind
+        if kind == L.KIND_PEP:
+            total = self._full_rows * inner._hidden_size
+            n = self.get_num_params()
+            return ((1 - n / total), n) if get_n_params else 1 - n / total
+        if kind == L.KIND_OPTEMBED or isinstance(inner, RetrainOptEmbed):
+            n = self._optembed_count() if kind == L.KIND_OPTEMBED else self.get_num_params()
+            sparsity = 1 - n / (inner._num_item * inner._hidden_size)
+            return (sparsity, n) if get_n_params else sparsity
+        return inner.get_sparsity(get_n_params)
+
+    @torch.no_grad()
+    def get_mask_e(self) -> torch.Tensor:
+        """OptEmbed.get_mask_e: [N] int64 on the CPU, 1 where a row survives mask-E; per shard, then all-gathered."""
+        inner = self.inner
+        if isinstance(inner._mask_e_module, nn.Identity):
+            return torch.ones(inner._num_item, dtype=torch.int64)
+        emb, _ = RF.optembed_eval_weight(inner._weight.detach(), self._shard_rows(inner._t_rows()), None, inner._norm)
+        local = (emb.abs().sum(1) > 0).to(torch.int64)
+        return self._gather_full(local, self._full_rows).cpu()
+
+    def get_submask(self) -> torch.Tensor:
+        """OptEmbed.get_submask from the global mask-E, cached on the wrapped module until the next training forward."""
+        inner = self.inner
+        if inner._submask_cache is None:
+            inner._submask_cache = inner._submask(self.get_mask_e)
+        return inner._submask_cache
 
     def train_callback(self):
         """PepEmbeeding.train_callback (pep_embedding.py:132-147) on the global sparsity: when a target is crossed every
@@ -668,17 +863,35 @@ class ShardedEmbedding(IEmbedding):
                 torch.save(state, os.path.join(inner.checkpoint_weight_dir, f"{target}.pth"))
             inner._cur_min_spar_idx += 1
 
-    def lookup(self, x, offsets=None, fc=None, bias=None):
+    def lookup(self, x, offsets=None, fc=None, bias=None, mask_d=None):
+        """The fused lookup over the shards.  `mask_d` is OptEmbed's: used outside training only (see forward)."""
         inner = self.inner
         spec = inner._spec()
-        table, table1, aux = inner._tensors()
         if offsets is not None:
             offsets = offsets.reshape(-1).long()
         self._rsb_err_flag = self.shards.err_flag
+        mask_d_idx = None
+        if spec.kind == L.KIND_OPTEMBED:
+            if not self.training:
+                emb, y = self._eval_lookup(x, offsets, fc, bias, mask_d)
+                if self.validate:
+                    RF.check_index_errors(self)
+                return emb, y
+            if x.dim() != 2 or x.shape[1] != inner._num_field:
+                raise RuntimeError("OptEmbed training forward expects x of shape [B, num_field]")
+            # weights are about to change: drop the eval cache (the module's own backward hook never runs here)
+            self._eval_state = "stale"
+            inner._submask_cache = None
+            # the same draw as the single-device forward (one torch.randint over this rank's [B, F] lookups)
+            mask_d_idx = inner._mask_d_for(x.shape[0], x.shape[1], x.device)
+        table, table1, aux = _kernel_tensors(inner)
+        if isinstance(inner, RetrainOptEmbed):
+            assert aux is not None, "Mask is not initialized"
         presort = RF.EARLY_SORT and torch.is_grad_enabled() and table.requires_grad
         slots = RF.amax_slots_for(x.device)
         aux_rep = None if self._per_row_aux else aux
-        emb, y, _ = _ShardedKindLookup.apply(self.shards, spec, x, offsets, table, table1, aux_rep, fc, bias, presort, slots)
+        emb, y, _ = _ShardedKindLookup.apply(self.shards, spec, x, offsets, table, table1, aux_rep, fc, bias, presort,
+                                             slots, mask_d_idx)
         if slots is not None:
             emb._rsb_amax_slots = slots
         if self.validate:
@@ -735,7 +948,7 @@ def _sharded_embedding(embedding_config, field_dims, num_factor, field_name, gro
 
 class ShardedDeepFM(_ShardedStepMixin, DeepFM):
     """DeepFM (src/models/deepfm.py:11-105) with the embedding's big arrays row-sharded (vanilla table, QR emb2, PEP
-    weight + thresholds, retrain weight + mask); the first-order weights `fc` (4 B per row), the MLP, `_bias` and
+    weight + thresholds, OptEmbed weight, retrain weight + mask); the first-order weights `fc` (4 B per row), the MLP, `_bias` and
     BatchNorm are replicated (BatchNorm statistics stay per-rank).  Build it after `dist.init_process_group` with the
     device current and the same seed on every rank."""
 
